@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the B200-native Unicorn per-frame hot path (contract: see the task statement / DESIGN.md §Measurement).
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--size H W]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--config NAME] [--size H W] [--dump-outputs DIR]
 
 A step = one steady-state SOT frame (BASELINE.json configs[1]: unicorn_track_large, 800x1280): backbone+neck ->
 deformable interaction -> 2x embedding upsample -> fused correlation/propagation -> head -> NMS, on synthetic video
@@ -9,6 +9,9 @@ with seeded random weights.  `value` = frames/s with frames resident in HBM (CUD
 `e2e` = frames/s through UnicornSOTTrack.track_tensor with pinned HOST frames (H2D + D2H inside the timed region).
 `--impl reference` times the reference algorithm's CPU restatement (oracle/, validated against the real reference)
 on the host cores for the same workload.
+Every frames/s figure of either impl times exactly `--steps` frames; only the kernel microbenchmarks and the `cpu_baseline`
+sample have fixed counts of their own.  Inputs and weights are seeded, so `--dump-outputs` of two builds run with
+the same arguments can be compared array for array.
 """
 import argparse
 import json
@@ -18,6 +21,7 @@ import sys
 import threading
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -103,7 +107,7 @@ def run_reference(args):
     cores = host_threads()
     torch.set_num_threads(cores)
     H, W = args.size
-    steps, warm = min(args.steps, 6), min(args.warmup, 1)
+    steps, warm = args.steps, min(args.warmup, 1)
     sd = make_state_dict(args.config, 0)
     frames, boxes = make_video(steps + warm + 1, H, W, seed=0)
     o = orc.SOTOracle(sd, args.config)
@@ -301,6 +305,17 @@ def pk_burst():
     return peaks()["tf_burst"]
 
 
+def last_step_outputs(ctx, max_inst):
+    """Host copies of what one SOT frame of an engine context produced: the detections collect() hands back (`dets`, rows
+    x1 y1 x2 y2 obj_conf cls_conf cls; `count`, the number NMS kept) and the dense maps behind them that the tracker exposes
+    as `last` (`head`, the decoded [A, 6] predictions; `priors`, the stride-8 label map propagated by the correlation)."""
+    n = int(ctx.ws.count.item())
+    out = {"dets": ctx.ws.dets[:min(n, max_inst)], "head": ctx.last["head"][0], "priors": ctx.last["priors"][0]}
+    out = {k: v.float().cpu().numpy() for k, v in out.items()}
+    out["count"] = np.array([n], dtype=np.float64)
+    return out
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -313,10 +328,14 @@ def main():
     ap.add_argument("--depth", type=int, default=3, help="frames in flight of the headline measurement (>= 2; the sequential numbers are always reported too)")
     ap.add_argument("--no-extra", action="store_true", help="skip the configs[2] (MOT 1536x2048) and configs[3] (VOS mask) workloads")
     ap.add_argument("--save-tuning", default=None, help="directory: write every engine's per-layer N-tile table (with UC_NO_TUNED=1: fresh autotuning)")
+    ap.add_argument("--dump-outputs", default=None, metavar="DIR",
+                    help="write the outputs of the headline measurement's last timed frame as DIR/<name>.npy (rank 0)")
     args = ap.parse_args()
     if args.size is None:
         args.size = (320, 320) if "tiny" in args.config else (800, 1280)
     if args.impl == "reference":
+        if args.dump_outputs:
+            ap.error("--dump-outputs applies to --impl ours")
         return run_reference(args)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -398,6 +417,8 @@ def main():
         return pipe, e0.elapsed_time(e1) / 1e3
     D = max(2, args.depth)
     pipe, dt_dev_pipe = measure_pipe(D)
+    # timed step i ran on context i % D; the later measurements reuse these buffers, so copy the last step's results now
+    dumped = last_step_outputs(pipe._ctxs[(K - 1) % D], pipe.max_inst) if args.dump_outputs and rank == 0 else None
     dt_dev_pipe3 = measure_pipe(D + 1)[1]
     # ---------------- end to end through the public API with pinned host frames, driven by the product's multi-GPU module:
     # one sequence per rank (parallel.shard_sequences), start barrier, wall clock of the slowest rank, one all_gather of the
@@ -524,7 +545,7 @@ def main():
                             "~26 us, not the tensor pipe; the separate kernels it replaces take 120 us (profiles/r2_mlp_fused_microbench.txt)",
                     "peak_source": "measured bf16_tflops (burst)"}
 
-    extra = {} if args.no_extra else extra_workloads(dev, rank, world, max(8, min(K, 24)), sync_all, args.save_tuning if rank == 0 else None)
+    extra = {} if args.no_extra else extra_workloads(dev, rank, world, K, sync_all, args.save_tuning if rank == 0 else None)
     if args.save_tuning and rank == 0:
         eng.save_tuning(os.path.join(args.save_tuning, f"{args.config}.json"))
     RI_frame = RI.get("frame", {})
@@ -592,6 +613,10 @@ def main():
     else:
         out["cpu_baseline"] = {"value": None, "unit": "frames/s", "cores": os.cpu_count(), "kind": "port", "sample": "skipped (N>1 or --no-cpu-baseline)"}
         out["cpu_baseline"]["cores"] = host_threads()
+    if dumped is not None:
+        os.makedirs(args.dump_outputs, exist_ok=True)
+        for name, a in dumped.items():
+            np.save(os.path.join(args.dump_outputs, f"{name}.npy"), a)
     print(json.dumps(out))
     if world > 1:
         dist.destroy_process_group()

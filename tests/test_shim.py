@@ -1,7 +1,8 @@
-"""The `unicorn`-importable shim (unicorn_b200/shim): API surface on CPU, and — in the build container, where /root/reference
-exists — the UNMODIFIED reference tracker file external/lib/test/tracker/unicorn_sot.py bound to the shim: it must import, walk
-its own __init__ (get_exp -> get_model -> torch.load -> load_state_dict) and stop exactly where the GPU is needed (`.cuda()`),
-with this package's loud no-fallback error."""
+"""The `unicorn`-importable shim (unicorn_b200/shim): API surface on CPU, and the UNMODIFIED reference tracker file
+external/lib/test/tracker/unicorn_sot.py bound to the shim through its recorded use of the package (tests/golden/shim_sot_api.json,
+written by tests/golden/make_golden_shim_api.py): its imports must resolve, its own __init__ sequence (get_exp -> get_model ->
+torch.load -> load_state_dict) must run and stop exactly where the GPU is needed (`.cuda()`), with this package's loud
+no-fallback error."""
 import os
 import subprocess
 import sys
@@ -11,7 +12,7 @@ import pytest
 import torch
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
+API = os.path.join(ROOT, "tests", "golden", "shim_sot_api.json")
 
 
 def test_shim_surface():
@@ -64,29 +65,42 @@ def test_shim_surface():
     assert r.returncode == 0 and "shim surface ok" in r.stdout, r.stdout + r.stderr
 
 
-@pytest.mark.skipif(not os.path.isdir(REF), reason="the reference checkout exists only in the build container")
 @pytest.mark.skipif(torch.cuda.is_available(), reason="on a GPU box the same flow runs to completion in tests/test_shim_gpu.py")
 def test_unmodified_reference_sot_tracker_binds_to_shim(tmp_path):
     code = textwrap.dedent(f"""
-        import sys, types
+        import importlib, json, sys
         sys.path.insert(0, {ROOT!r})
         import unicorn_b200.shim as shim
         shim.install()                                   # `unicorn` -> unicorn_b200/shim/unicorn
-        sys.path.insert(1, {REF + '/external'!r})          # lib.test.tracker.* : the reference's own, unmodified files
         import torch
         from unicorn_b200.weights import make_state_dict
         from unicorn_b200._lib import UnicornB200Error
-        import lib.test.tracker.unicorn_sot as ref_sot
-        assert ref_sot.__file__.startswith({REF!r}) and sys.modules["unicorn"].__unicorn_b200_shim__
-        assert ref_sot.postprocess.__module__ == "unicorn_b200.compat.model"
+        api = json.load(open({API!r}))
+        names = {{}}
+        for mod, name in api["imports"]:                 # the tracker file's `from unicorn... import ...` lines
+            m = importlib.import_module(mod)
+            assert m.__file__.startswith({os.path.join(ROOT, "unicorn_b200")!r}), (mod, m.__file__)
+            names[name] = getattr(m, name)
+        assert sys.modules["unicorn"].__unicorn_b200_shim__
+        assert names["postprocess"].__module__ == "unicorn_b200.compat.model"
         ckpt = {str(tmp_path / 'c.pth')!r}
-        torch.save({{"model": make_state_dict("unicorn_track_tiny", 0)}}, ckpt)
-        params = types.SimpleNamespace(exp_name="unicorn_track_tiny", checkpoint=ckpt)
-        try:
-            ref_sot.UnicornSOTTrack(params, "lasot")
+        torch.save({{api["checkpoint_key"]: make_state_dict("unicorn_track_tiny", 0)}}, ckpt)
+        exp = names["get_exp"](api["get_exp_file"] % "unicorn_track_tiny", None)
+        for a in api["exp_attributes"]:
+            getattr(exp, a)
+        model = exp.get_model(**api["get_model_kwargs"])
+        missing = [a for a in api["model_attributes"] if not hasattr(model, a)]
+        assert not missing, missing
+        sd = torch.load(ckpt, map_location="cpu")[api["checkpoint_key"]]
+        for meth, kw in api["init_model_calls"]:
+            try:
+                getattr(model, meth)(*((sd,) if meth == "load_state_dict" else ()), **kw)
+            except UnicornB200Error as e:                # raised by self.model.cuda(): no CPU fallback
+                assert meth == "cuda", meth
+                print("stopped at .cuda():", str(e)[:80])
+                break
+        else:
             raise SystemExit("constructed without a GPU")
-        except UnicornB200Error as e:                    # raised by self.model.cuda() (unicorn_sot.py:29): no CPU fallback
-            print("stopped at .cuda():", str(e)[:80])
         print("reference tracker bound ok")
     """)
     r = subprocess.run([sys.executable, "-c", code], capture_output=True, text=True, timeout=600)

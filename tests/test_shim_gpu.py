@@ -1,20 +1,13 @@
 """The `unicorn` shim on the GPU: a tracker written against the REFERENCE'S API only (`from unicorn.exp import get_exp`,
 `model(..., mode=...)`, `model.head(...)`, `unicorn.utils.boxes.postprocess`; the call sequence of
 external/lib/test/tracker/unicorn_sot.py:26-109, torch fp16 mm + softmax(dim=0) correlation included) must produce the boxes of the
-product driver UnicornSOTTrack.  If the reference checkout is present (it is not on the GPU box) its own unmodified tracker class
-is driven instead of the restated flow.  Mask model: shim postprocess_inst against the kernels' direct result."""
-import os
-import sys
-import types
-
+product driver UnicornSOTTrack.  Mask model: shim postprocess_inst against the kernels' direct result."""
 import numpy as np
 import pytest
 import torch
 import torch.nn.functional as F
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-REF = "/root/reference"
 
 
 @pytest.fixture(scope="module")
@@ -95,23 +88,13 @@ def test_api_only_tracker_matches_product_driver(shim, tmp_path):
     ckpt = str(tmp_path / "ckpt.pth")
     torch.save({"model": sd}, ckpt)
     rgb, xywh = _rgb_frames(6, 256, 400, seed=9)
-    if os.path.isdir(REF):  # the reference's own, unmodified tracker class on top of the shim
-        sys.path.insert(1, os.path.join(REF, "external"))
-        np.int = int  # numpy >= 1.24 (unicorn_sot.py:74 uses the removed alias)
-        from lib.test.tracker.unicorn_sot import UnicornSOTTrack as RefTrack
-        a = RefTrack(types.SimpleNamespace(exp_name=name, checkpoint=ckpt), "lasot")
-        a.input_size = size
-        a.initialize(rgb[0], {"init_bbox": xywh[0].tolist()})
-        track_a = lambda im: a.track(im)["target_bbox"]  # noqa: E731
-    else:
-        a = ApiOnlySOT(name, ckpt, size)
-        a.initialize(rgb[0], xywh[0].tolist())
-        track_a = lambda im: a.track(im)["target_bbox"]  # noqa: E731
+    a = ApiOnlySOT(name, ckpt, size)
+    a.initialize(rgb[0], xywh[0].tolist())
     b = UnicornSOTTrack(UnicornEngine(sd, name), size, use_graph=True)
     b.initialize(rgb[0], {"init_bbox": xywh[0].tolist()})
     diffs = []
     for t in range(1, 6):
-        sa, sb = track_a(rgb[t]), b.track(rgb[t])["target_bbox"]
+        sa, sb = a.track(rgb[t])["target_bbox"], b.track(rgb[t])["target_bbox"]
         diffs.append(np.abs(np.array(sa, dtype=np.float32) - np.array(sb, dtype=np.float32)).max())
     print("API-only tracker vs UnicornSOTTrack, max |box difference| per frame (pixels):", diffs)
     # same engine kernels; the only difference is the unfused fp16 correlation of the reference flow vs the fused kernel
