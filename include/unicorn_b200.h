@@ -248,6 +248,21 @@ typedef struct UcVosObject {
 UC_API int uc_vos_aggregate(const UcVosObject* objs, int n, int Hin, int Win, int H, int W, float r, float* soft_out,
                             uint8_t* seg_out, void* stream);
 
+/* MOTS mask tail on the device (unicorn/evaluators/mot_evaluator.py:804-805 resize + threshold, :858-866 overlap free, :882-888
+ * area filter + COCO RLE): masks f32 [n_max, Hin, Win] (uc_dynamic_masks output); rows device int32 [K] = the mask rows in
+ * output order (ascending track id); emit device int32 [K] = 1 for the rows that pass the area filter.  Every row is resized
+ * with F.interpolate(scale_factor, bilinear, align_corners=False) — output floor(Hin * scale_factor) x floor(Win * scale_factor)
+ * computed in double, source scale (float)(1 / scale_factor) —, cropped to [:img_h, :img_w], thresholded (value > thres) and
+ * keeps only the pixels no earlier row of `rows` claimed (rows with emit = 0 claim too).  Each emitted row is encoded as the
+ * COCO compressed RLE string of its column-major mask (byte-identical to unicorn_b200.results.rle_encode).
+ * Outputs (device): out_len[k] = string length (0 when not emitted), out_off[k] = its offset in out_chars, *out_total = the sum
+ * of the lengths.  Strings are written only where they fit in `capacity` bytes; when *out_total > capacity, run again with a
+ * larger buffer.  workspace >= uc_mots_rle_workspace_bytes(K, Hin, Win, img_h, img_w, scale_factor) bytes (0 = bad sizes). */
+UC_API long uc_mots_rle_workspace_bytes(int K, int Hin, int Win, int img_h, int img_w, double scale_factor);
+UC_API int uc_mots_masks_rle(const float* masks, int n_max, int Hin, int Win, const int* rows, const int* emit, int K, int img_h,
+                             int img_w, float thres, double scale_factor, void* workspace, long workspace_bytes, long long* out_len,
+                             long long* out_off, long long* out_total, char* out_chars, long capacity, void* stream);
+
 #ifdef __cplusplus
 }
 #endif

@@ -427,3 +427,47 @@ def dynamic_masks(mask_feats, up_masks, dyn_levels, level_hw, ws, n_max, up_rate
     _lib.check(_L().uc_dynamic_masks(_p(mask_feats), _p(up_masks), h, w, up_rate, d_rate, dl, dyn_levels[0].shape[-1], hw, st, so,
                                      _p(ws.anchors), _p(ws.count), n_max, _p(scratch), _p(out), _S()), "uc_dynamic_masks", 3)
     return out
+
+
+class MotsRleWorkspace:
+    """Device buffers of mots_masks_rle: bit-packed masks, per-row lengths / offsets and the string bytes.  Allocated on first use
+    and grown when a frame needs more (the string buffer when the kernel reports that the strings did not fit)."""
+
+    def __init__(self, device, capacity=1 << 16):
+        self.dev = torch.device(device)
+        self.bits = torch.empty(0, dtype=torch.uint8, device=self.dev)
+        self.meta = torch.empty(0, dtype=torch.int64, device=self.dev)
+        self.chars = torch.empty(capacity, dtype=torch.uint8, device=self.dev)
+
+
+def mots_masks_rle(masks, rows, emit, img_h, img_w, thres, scale_factor, ws=None):
+    """COCO RLE strings of the MOTS masks of one frame (uc_mots_masks_rle): masks fp32 [n_max, Hin, Win] (device); rows / emit int32
+    [K] device tensors (mask rows in ascending track-id order, area-filter flags).  Row k is resized with F.interpolate(scale_factor,
+    bilinear, align_corners=False)[:img_h, :img_w], thresholded (> thres) and made overlap free against rows 0..k-1.  Returns the
+    strings of the emitted rows, in order; only the lengths and the string bytes are copied to the host."""
+    K = rows.numel()
+    if K == 0:
+        return []
+    n_max, Hin, Win = masks.shape
+    assert masks.dtype == torch.float32 and masks.is_contiguous() and masks.is_cuda
+    assert rows.dtype == torch.int32 and emit.dtype == torch.int32 and emit.numel() == K and rows.is_cuda and emit.is_cuda
+    ws = ws or MotsRleWorkspace(masks.device)
+    fn = _L().uc_mots_rle_workspace_bytes
+    fn.restype = ctypes.c_long
+    need = fn(K, Hin, Win, img_h, img_w, ctypes.c_double(scale_factor))
+    if need > ws.bits.numel():
+        ws.bits = torch.empty(need, dtype=torch.uint8, device=masks.device)
+    if ws.meta.numel() < 2 * K + 1:
+        ws.meta = torch.empty(2 * K + 1, dtype=torch.int64, device=masks.device)
+    while True:
+        meta = ws.meta[:2 * K + 1]
+        _lib.check(_L().uc_mots_masks_rle(_p(masks), n_max, Hin, Win, _p(rows), _p(emit), K, img_h, img_w, _f(thres), ctypes.c_double(scale_factor),
+                                          _p(ws.bits), _l(ws.bits.numel()), _p(meta), _p(meta[K:]), _p(meta[2 * K:]), _p(ws.chars),
+                                          _l(ws.chars.numel()), _S()), "uc_mots_masks_rle", 3)
+        m = meta.cpu().tolist()
+        total = m[2 * K]
+        if total <= ws.chars.numel():
+            break
+        ws.chars = torch.empty(max(total, 2 * ws.chars.numel()), dtype=torch.uint8, device=masks.device)  # run again, never truncate
+    data = ws.chars[:total].cpu().numpy().tobytes()
+    return [data[m[K + k]:m[K + k] + m[k]].decode("ascii") for k in range(K) if m[k] > 0]
